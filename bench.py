@@ -21,10 +21,13 @@ scenarios per GPU, replicas, no gather) is reported under extra.weak.
 """
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -70,10 +73,18 @@ def vel_kwargs():
     return dict(vel_max=100.0, gg_scale=1.0, local_gg=(5.0, 5.0), ax_max_machines=ax_max_machines(), safety_d=30.0)
 
 
+_CACHE_DIR = []
+
+
 def lattice_cache_path(tag):
-    d = os.path.join(REPO, ".lattice_cache")
-    os.makedirs(d, exist_ok=True)
-    return os.path.join(d, "lattice_%s.npz" % tag)
+    """The CPU workers load the lattice from this file, so it must be written somewhere writable even when the tree is
+    read-only.  It is written fresh in a directory of this run: the cache key covers the input files but not the code,
+    so a file left by another build could be stale.  Every run therefore builds its lattices anew, outside the timed
+    regions."""
+    if not _CACHE_DIR:
+        _CACHE_DIR.append(tempfile.mkdtemp(prefix="ltpl_bench_"))
+        atexit.register(shutil.rmtree, _CACHE_DIR[0], True)
+    return os.path.join(_CACHE_DIR[0], "lattice_%s.npz" % tag)
 
 
 def get_lattice(tag):
@@ -281,6 +292,46 @@ def algorithmic_bytes(lat, stats):
                 k_vel_fp32_sizes=vel_fp32, tick_survey_8d=b_tick)
 
 
+DUMP_BYTES = 64 << 20
+DUMP_SAMPLE = 1024
+
+
+def dump_outputs(pl, out_dir, seed=SEED):
+    """The result of the planner's last tick as out_dir/<name>.npy: the per-path arrays of every scenario ([slot, B] or
+    [B, ...]) and, for a fixed seeded sample of scenarios (sample.npy), the paths, node sequences, f64 trajectories
+    (s, vx, ax) and exported f32 trajectory rows, indexed [slot, sample, ...] and zeroed past their lengths.  Exported
+    rows are looked up through traj_row: the kernels claim them in a run-dependent order.  Everything is float64 except
+    the exported rows (float32), at most DUMP_BYTES in all."""
+    from graphbasedlocaltrajectoryplanner_b200 import capi
+    f = pl.fetch("sc_flags", "start_node", "closest_obj", "action_id", "status", "path_len", "n_nodes", "traj_len",
+                 "traj_id", "nodes", "node_idx", "path", "s_vx_ax", "traj", "traj_row")
+    out = {k: f[k].astype(np.float64) for k in ("sc_flags", "start_node", "closest_obj", "action_id", "status",
+                                                "path_len", "n_nodes", "traj_len", "traj_id")}
+    B = pl.dims.batch
+    nslot, _, H, _ = f["nodes"].shape
+    P, NE = f["path"].shape[2], f["traj"].shape[1]
+    per_scenario = nslot * (8 * P * (5 + 3) + 8 * H * (2 + 1) + 4 * NE * 7) + 8
+    n = min(B, DUMP_SAMPLE, (DUMP_BYTES - sum(v.nbytes for v in out.values())) // per_scenario)
+    idx = np.sort(np.random.default_rng(seed).choice(B, n, replace=False))
+    q = np.arange(nslot)[:, None] * B + idx[None, :]                      # [slot, sample] -> row of path / s_vx_ax
+    planned = f["action_id"][:, idx] != capi.ACT_NONE
+    valid = planned & ((f["status"][:, idx] & capi.ST_TRAJ_VALID) != 0) & (f["traj_row"][:, idx] >= 0)
+    on_path = (planned[..., None] & (np.arange(P) < f["path_len"][:, idx][..., None]))[..., None]
+    on_traj = (valid[..., None] & (np.arange(P) < f["path_len"][:, idx][..., None]))[..., None]
+    on_nodes = planned[..., None] & (np.arange(H) < f["n_nodes"][:, idx][..., None])
+    on_rows = (valid[..., None] & (np.arange(NE) < f["traj_len"][:, idx][..., None]))[..., None]
+    out["sample"] = idx.astype(np.float64)
+    out["path"] = np.where(on_path, f["path"][:, q].transpose(1, 2, 3, 0), 0.0)
+    out["s_vx_ax"] = np.where(on_traj, f["s_vx_ax"][:, q].transpose(1, 2, 3, 0), 0.0)
+    out["nodes"] = np.where(on_nodes[..., None], f["nodes"][:, idx], -1).astype(np.float64)
+    out["node_idx"] = np.where(on_nodes, f["node_idx"][:, idx], -1).astype(np.float64)
+    out["traj"] = np.where(on_rows, f["traj"][np.where(valid, f["traj_row"][:, idx], 0)], np.float32(0.0))
+    assert sum(v.nbytes for v in out.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -293,7 +344,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra lines (other lattices, stateful tick, config 5, weak)")
     ap.add_argument("--no-peer", action="store_true", help="multi-GPU gather by point-to-point sends instead of peer stores")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy (--gpus 1)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.gpus > 1 or args.impl != "b200"):
+        ap.error("--dump-outputs writes the result of the GPU tick of --gpus 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -443,6 +498,8 @@ def main():
     barrier()
     t_dev = max_over_ranks(t_dev)
     value = args.batch * args.steps / t_dev
+    if args.dump_outputs:
+        dump_outputs(pl, args.dump_outputs)
     gathered_rows = None
     if world > 1 and rank == 0 and gather is not None:   # the consumer sees every rank's rows: count them
         gathered_rows = 0

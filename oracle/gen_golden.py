@@ -31,7 +31,8 @@ ACTIONS = ("straight", "follow", "left", "right")
 
 def load_reference(use_shims=True):
     """import the reference package on top of the shims (use_shims=False: on REAL python-igraph /
-    trajectory_planning_helpers installs, tests/test_against_reference.py); returns the `graph_ltpl` module."""
+    trajectory_planning_helpers installs, to compare the reference on them with the stored fixtures); returns the
+    `graph_ltpl` module."""
     if not os.path.isdir(REF):
         raise RuntimeError("/root/reference is not available on this box")
     for p in ((REPO, os.path.join(REPO, 'oracle', 'shims'), REF) if use_shims else (REPO, REF)):
@@ -448,6 +449,30 @@ def variants_fixture(graph_ltpl, track, n):
     return out
 
 
+SEED86420 = (("default", {}, 48, 0, 3), ("l216", {"lat_resolution": 1.0, "lon_straight_step": 12.0}, 24, 1, 3))
+SEED86420_STRIDE = 4
+
+
+def seed86420_fixture(graph_ltpl, track, tag, overrides, n, omin, omax, vel_kwargs):
+    """first ticks of the seed-86420 scenarios of tests/test_against_reference.py: the arrays H.compare_record reads
+    (no spline coefficients) and the scenario inputs.  To keep the file small, paths and trajectories keep every
+    SEED86420_STRIDE-th point (point_stride) in float32 (relative rounding 6e-8, the comparison tolerance is 1e-4)."""
+    from graphbasedlocaltrajectoryplanner_b200.scenarios import make_scenarios
+    ltpl, _ = make_ltpl(graph_ltpl, tag, overrides)
+    sc = make_scenarios(track, n, seed=86420, n_obj_min=omin, n_obj_max=omax)
+    recs = [run_tick(ltpl, sc.pos[b], sc.heading[b], sc.vel[b], sc.object_list(b), vel_kwargs, full=True)
+            for b in range(sc.size)]
+    pk = pack_ticks(recs)
+    del pk['coeff'], pk['coeff_len']
+    for k in ('path', 'traj'):
+        pk[k] = pk[k][:, :, ::SEED86420_STRIDE].astype(np.float32)
+    payload = {('full_' + k): v for k, v in pk.items()}
+    payload['point_stride'] = np.int32(SEED86420_STRIDE)
+    payload.update(sc_pos=sc.pos, sc_heading=sc.heading, sc_vel=sc.vel, sc_n_obj=sc.n_obj, sc_obj=sc.obj,
+                   ax_max_machines=vel_kwargs['ax_max_machines'], overrides=np.array(repr(sorted(overrides.items()))))
+    return payload
+
+
 def lattice_fixture(graph_ltpl, ltpl, n_edge_samples=300, seed=7):
     """compact description of the reference-built GraphBase (validates the product's lattice builder)."""
     from graphbasedlocaltrajectoryplanner_b200.lattice import Lattice
@@ -493,6 +518,7 @@ def main():
     ap.add_argument('--variants-only', action='store_true', help='only the parameter-variant fixture')
     ap.add_argument('--n-variant', type=int, default=24)
     ap.add_argument('--ggpp-only', action='store_true', help='only the location dependent local_gg fixtures')
+    ap.add_argument('--seed86420-only', action='store_true', help='only the fixtures of tests/test_against_reference.py')
     args = ap.parse_args()
 
     graph_ltpl = load_reference()
@@ -502,6 +528,11 @@ def main():
     vel_kwargs = dict(vel_max=100.0, gg_scale=1.0, local_gg=(5.0, 5.0), ax_max_machines=ax_max_machines_table(),
                       safety_d=30.0, incl_emerg_traj=False)
 
+    if args.seed86420_only:
+        for tag, overrides, n, omin, omax in SEED86420:
+            np.savez_compressed(os.path.join(GOLDEN, 'ticks_seed86420_%s.npz' % tag),
+                                **seed86420_fixture(graph_ltpl, track, tag, overrides, n, omin, omax, vel_kwargs))
+        return
     if args.ggpp_only:
         # location dependent friction: local_gg = {action: [ndarray(P, 2)]} (OTH:649-666, VPFB:194-227), emergency
         # trajectory on (its brake profile takes the raw local_gg of the base trajectory, OTH:1030); closed loop with a grip

@@ -72,8 +72,11 @@ def assert_close(name, got, want, cols, ctx="", w_rel=None):
 
 
 def compare_record(rec, g, b, prefix="full_", ctx=""):
-    """compare one tick record (dict of dicts like oracle.tick()) against row b of a golden ticks file."""
+    """compare one tick record (dict of dicts like oracle.tick()) against row b of a golden ticks file.  A file with
+    `point_stride` s stores every s-th point of the paths and trajectories; path_len / traj_len stay the full lengths
+    and are compared exactly."""
     ctx = "%s scenario %d" % (ctx, b)
+    s = int(g["point_stride"]) if "point_stride" in g.files else 1
     assert bool(rec["out_of_track"]) == bool(g[prefix + "out_of_track"][b]), ctx
     if rec["out_of_track"]:
         return
@@ -92,7 +95,9 @@ def compare_record(rec, g, b, prefix="full_", ctx=""):
             ni = np.asarray(rec["node_idx"][act][0]).tolist()
             assert ni == g[prefix + "node_idx"][b, a, :len(ni)].tolist(), ctx + " node_idx " + act
             assert bool(rec["red_len"][act][0]) == bool(g[prefix + "red_len"][b, a]), ctx + " red_len " + act
-            assert_close("path[%s]" % act, rec["paths"][act][0], g[prefix + "path"][b, a, :n_want],
+            assert len(rec["paths"][act][0]) == n_want, "%s: path %s has %d points, golden %d" % (
+                ctx, act, len(rec["paths"][act][0]), n_want)
+            assert_close("path[%s]" % act, rec["paths"][act][0][::s], g[prefix + "path"][b, a, :(n_want + s - 1) // s],
                          ("x", "y", "psi", "kappa", "el"), ctx)
         t_want = int(g[prefix + "traj_len"][b, a])
         t_has = act in rec["traj_full"] and len(rec["traj_full"][act]) > 0
@@ -100,7 +105,9 @@ def compare_record(rec, g, b, prefix="full_", ctx=""):
         if t_has:
             # the id base (+10 per calc_vel_profile call, OTH:669) is instance state; the action code is id % 10
             assert int(rec["ids"][act]) % 10 == int(g[prefix + "traj_id"][b, a]) % 10, ctx + " traj id " + act
-            assert_close("traj[%s]" % act, rec["traj_full"][act][0], g[prefix + "traj"][b, a, :t_want],
+            assert len(rec["traj_full"][act][0]) == t_want, "%s: trajectory %s has %d points, golden %d" % (
+                ctx, act, len(rec["traj_full"][act][0]), t_want)
+            assert_close("traj[%s]" % act, rec["traj_full"][act][0][::s], g[prefix + "traj"][b, a, :(t_want + s - 1) // s],
                          ("s", "x", "y", "psi", "kappa", "vx", "ax"), ctx)
             assert rec["traj"][act][0].shape[0] == int(g["cut_traj_len"][b, a]) if "cut_traj_len" in g.files else True
 

@@ -1,69 +1,26 @@
-"""Differential test against the unmodified reference on REAL third-party installs (SURVEY 4(iv)).
+"""Differential test of the oracle against the unmodified reference on the scenarios of seed 86420.
 
-The golden vectors of this repository were produced by the reference's own files running on restatements of its two
-un-vendored dependencies (oracle/shims: igraph, trajectory_planning_helpers = oracle/tph_port.py), because neither
-python-igraph==0.8.2 nor trajectory_planning_helpers==0.75 is installable offline.  What stays unpinned by that is the
-third-party arithmetic itself (tph functions, igraph's heap order on exact ties).  On a box that HAS both packages and
-the reference checkout this test closes the gap: it runs the reference on the real packages and compares the oracle
-(CPU) with it, scenario by scenario, with the tolerances of the parity suite.  Everywhere else it is skipped."""
-import importlib.util
-import os
-import sys
-
-import numpy as np
+The expected arrays are the reference's own output (graph_ltpl @ 18763ef9, one first tick per scenario through its
+public API), produced by ``python -m oracle.gen_golden --seed86420-only`` and stored as
+tests/golden/ticks_seed86420_<tag>.npz, so the comparison needs neither the reference checkout nor its dependencies.
+python-igraph==0.8.2 and trajectory_planning_helpers==0.75 are not installable offline, so the reference ran on their
+restatements under oracle/shims; what stays unpinned by that is the third-party arithmetic itself (tph functions,
+igraph's heap order on exact ties)."""
 import pytest
 
 from tests import helpers as H
 
-REF = "/root/reference"
-
-
-def _real(mod):
-    """a real install of `mod` (not the restatement under oracle/shims)?"""
-    shim_dir = os.path.join(H.REPO, "oracle", "shims")
-    keep = list(sys.path)
-    try:
-        sys.path = [p for p in sys.path if os.path.abspath(p or ".") != shim_dir]
-        spec = importlib.util.find_spec(mod)
-    except (ImportError, ValueError):
-        spec = None
-    finally:
-        sys.path = keep
-    return spec is not None and spec.origin is not None and not os.path.abspath(spec.origin).startswith(shim_dir)
-
-
-pytestmark = pytest.mark.skipif(
-    not (os.path.isdir(REF) and _real("igraph") and _real("trajectory_planning_helpers")),
-    reason="needs /root/reference plus real python-igraph and trajectory_planning_helpers installs (offline: absent)")
-
 
 @pytest.mark.parametrize("tag,n,omin,omax", [("default", 48, 0, 3), ("l216", 24, 1, 3)])
-def test_oracle_matches_reference_on_real_igraph_and_tph(tag, n, omin, omax):
-    import ast
-    from graphbasedlocaltrajectoryplanner_b200.scenarios import Track, make_scenarios
-    from oracle import gen_golden as G
+def test_oracle_matches_stored_reference_ticks(tag, n, omin, omax):
     from oracle.ltpl_oracle import OracleLTPL
-    graph_ltpl = G.load_reference(use_shims=False)
-    import igraph
-    import trajectory_planning_helpers as tph
-    assert "shims" not in igraph.__file__ and "shims" not in tph.__file__
-    ov = dict(ast.literal_eval(str(H.golden("ticks_%s.npz" % tag)["overrides"])))
-    ltpl, _ = G.make_ltpl(graph_ltpl, tag + "_real", ov)
-    vk = dict(vel_max=100.0, gg_scale=1.0, local_gg=(5.0, 5.0), ax_max_machines=G.ax_max_machines_table(), safety_d=30.0,
-              incl_emerg_traj=False)
+    g = H.golden("ticks_seed86420_%s.npz" % tag)
+    assert g["sc_pos"].shape[0] == n and omin <= g["sc_n_obj"].min() and g["sc_n_obj"].max() <= omax
+    vk = dict(vel_max=100.0, gg_scale=1.0, local_gg=(5.0, 5.0), ax_max_machines=g["ax_max_machines"], safety_d=30.0)
     orc = OracleLTPL(H.lattice_for(tag))
-    sc = make_scenarios(Track(H.TRACK_CSV), n, seed=86420, n_obj_min=omin, n_obj_max=omax)
-    recs = [G.run_tick(ltpl, sc.pos[b], sc.heading[b], sc.vel[b], sc.object_list(b), vk, full=True) for b in range(n)]
-    g = G.pack_ticks(recs)
-    g = {("full_" + k): v for k, v in g.items()}
-    g_files = type("G", (), {"files": list(g)})()
     compared = 0
     for b in range(n):
-        rec = orc.tick(sc.pos[b], sc.heading[b], sc.vel[b], sc.object_list(b), {k: v for k, v in vk.items()
-                                                                                 if k != "incl_emerg_traj"})
-
-        class _View(dict):
-            files = g_files.files
-        H.compare_record(rec, _View(g), b, ctx="real-deps " + tag)
+        rec = orc.tick(g["sc_pos"][b], g["sc_heading"][b], g["sc_vel"][b], H.object_list(g, b), vk)
+        H.compare_record(rec, g, b, ctx="seed86420 " + tag)
         compared += int(not rec["out_of_track"])
     assert compared > n // 2

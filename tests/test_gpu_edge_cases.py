@@ -89,11 +89,11 @@ def test_vel_max_below_planned_velocity_is_reported():
     assert np.all((f["sc_flags"][ok] & capi.SC_BRAKE_PREFIX) != 0) and int(f["traj_len"].sum()) == 0
 
 
-def test_single_scenario_facade_matches_config1_and_errors():
+def test_single_scenario_facade_matches_config1_and_errors(tmp_path):
     """Graph_LTPL facade with the reference's call sequence (main_min_example.py:69-104) + error behaviour."""
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     g = H.golden("config1_min_example.npz")
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     ltpl = Graph_LTPL(path_dict=pd, visual_mode=False, log_to_file=False, device="cuda:0")
     ltpl.graph_init()

@@ -17,19 +17,19 @@ class _Clock(object):
         return self.t
 
 
-def _path_dict():
+def _path_dict(tmp_path):
     # main_min_example.py:42-46 passes exactly these four entries (log_to_file=False needs no log paths, LTPL:62-68)
-    return {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    return {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
             'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
 
 
-def test_min_example_loop_runs_unchanged():
+def test_min_example_loop_runs_unchanged(tmp_path):
     """body of main_min_example.py:52-107 with the import swapped: graph_init, set_startpos at the first reference-line
     point, then the online loop (brute-force action choice, calc_paths, vehicle dummy, calc_vel_profile, visual)."""
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     from graphbasedlocaltrajectoryplanner_b200.lattice import import_globtraj_csv
     from oracle.gen_golden import advance_on_traj   # stands in for testing_tools/src/vdc_dummy.py (test infrastructure)
-    ltpl_obj = Graph_LTPL(path_dict=_path_dict(), visual_mode=True, log_to_file=False)
+    ltpl_obj = Graph_LTPL(path_dict=_path_dict(tmp_path), visual_mode=True, log_to_file=False)
     ltpl_obj.graph_init()
     refline = import_globtraj_csv(H.TRACK_CSV)["refline"]
     pos_est = refline[0, :]
@@ -59,7 +59,7 @@ def test_min_example_loop_runs_unchanged():
     assert s_driven > 0.0 and t[-1, 5] > t[0, 5] + 5.0   # the dummy moved; the plans accelerate away from standstill
 
 
-def test_session_with_growing_object_list_and_unknown_action():
+def test_session_with_growing_object_list_and_unknown_action(tmp_path):
     """one stateful session through the facade against the session oracle (pinned on the reference): the object list
     grows from 0 to 3 entries between ticks (the scenario input buffers are re-created, the device memory must
     survive), and one tick names an action the last tick did not return (OTH:393-407)."""
@@ -70,7 +70,7 @@ def test_session_with_growing_object_list_and_unknown_action():
     from oracle.ltpl_session import OracleSession
     g = H.golden("ticks_multitick_default.npz")
     vel = dict(vel_max=100.0, gg_scale=1.0, local_gg=(5.0, 5.0), ax_max_machines=g["ax_max_machines"], safety_d=30.0)
-    ltpl = Graph_LTPL(path_dict=_path_dict(), visual_mode=False, log_to_file=False, device="cuda:0")
+    ltpl = Graph_LTPL(path_dict=_path_dict(tmp_path), visual_mode=False, log_to_file=False, device="cuda:0")
     ltpl.graph_init()
     lat = H.lattice_for("default")
     sc = make_scenarios(Track(H.TRACK_CSV), 6, seed=4711, n_obj_min=3, n_obj_max=3)

@@ -265,13 +265,13 @@ def test_closed_loop_matches_session_oracle(tag, n_seq, omin, omax):
 
 @pytest.mark.parametrize("fixture,seqs,emerg", [("ticks_multitick_default.npz", (0, 5, 11), False),
                                                 ("ticks_multitick_emsel_default.npz", (1, 3), True)])
-def test_facade_runs_closed_loop_like_the_reference(fixture, seqs, emerg):
+def test_facade_runs_closed_loop_like_the_reference(fixture, seqs, emerg, tmp_path):
     """Graph_LTPL facade with the reference's call sequence over several ticks (main_std_example.py:99-126): an injected
     clock takes the place of time.time(); recorded sequences of the reference are replayed (second case: the caller
     executes the 'emergency' trajectory for three ticks, prev_action_id='emergency')."""
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     g = H.golden(fixture)
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     ltpl = Graph_LTPL(path_dict=pd, visual_mode=False, log_to_file=False, device="cuda:0")
     ltpl.graph_init()

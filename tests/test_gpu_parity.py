@@ -91,13 +91,13 @@ def test_cuda_matches_oracle_seeded(tag, n, omin, omax):
     assert not fails, "%d/%d scenarios differ from the oracle:\n%s" % (len(fails), sc.size, "\n".join(fails[:10]))
 
 
-def test_plan_stream_pipelining_matches_plan_batch():
+def test_plan_stream_pipelining_matches_plan_batch(tmp_path):
     """the pipelined end-to-end API (two export buffers, D2H overlapping the next step) returns, for every step, the
     same action sets as the synchronous plan_batch call."""
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     from graphbasedlocaltrajectoryplanner_b200.scenarios import Track, make_scenarios
     g = H.golden("ticks_default.npz")
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     ltpl = Graph_LTPL(path_dict=pd, log_to_file=False, device="cuda:0")
     ltpl.graph_init()

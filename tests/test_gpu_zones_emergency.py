@@ -96,10 +96,10 @@ def test_zones_and_emergency_match_oracle_seeded():
     assert n_em > sc.size // 2
 
 
-def test_facade_blocked_zones_and_emergency():
+def test_facade_blocked_zones_and_emergency(tmp_path):
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     g = H.golden("ticks_ext_default.npz")
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     ltpl = Graph_LTPL(path_dict=pd, visual_mode=False, log_to_file=False, device="cuda:0")
     ltpl.graph_init()
@@ -212,7 +212,7 @@ def test_explicit_predictions_match_reference_golden_and_oracle():
         H.compare_records(recs3[b], want, ctx="no-pred after pred %d" % b)
 
 
-def test_location_dependent_local_gg_matches_reference_golden():
+def test_location_dependent_local_gg_matches_reference_golden(tmp_path):
     """calc_vel_profile(local_gg={action: [ndarray(P, 2)]}) (OTH:649-666, VPFB:194-227) against the reference: friction
     as a function of the position along every path (buffers.gg planes, k_vel_res<.., GG>), emergency trajectory on
     (raw local_gg of its base trajectory, OTH:1030); batch API and the facade's dict form."""
@@ -242,7 +242,7 @@ def test_location_dependent_local_gg_matches_reference_golden():
             n_em += 1
     assert n_em >= sc.size // 2
     # the facade takes the reference's dict form
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_lat_default_test.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     ltpl = Graph_LTPL(path_dict=pd, visual_mode=False, log_to_file=False, device="cuda:0")
     ltpl.graph_init()

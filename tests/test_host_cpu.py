@@ -68,11 +68,11 @@ def test_scenarios_deterministic_and_in_track():
     assert np.allclose(rt.obj[0, :len(ol)], a.obj[0, :len(ol)])
 
 
-def test_facade_argument_checks():
+def test_facade_argument_checks(tmp_path):
     from graphbasedlocaltrajectoryplanner_b200.Graph_LTPL import Graph_LTPL
     with pytest.raises(ValueError):   # LTPL:62-68 missing path entries
         Graph_LTPL(path_dict={'globtraj_input_path': H.TRACK_CSV}, log_to_file=False)
-    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': "/tmp/_x.npz",
+    pd = {'globtraj_input_path': H.TRACK_CSV, 'graph_store_path': str(tmp_path / "lattice_default.npz"),
           'ltpl_offline_param_path': H.OFFLINE_INI, 'ltpl_online_param_path': H.ONLINE_INI}
     obj = Graph_LTPL(path_dict=pd, log_to_file=False)
     with pytest.raises(ValueError):   # LTPL:277-280 graph not initialised
