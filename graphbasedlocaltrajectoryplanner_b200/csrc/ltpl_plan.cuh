@@ -153,7 +153,8 @@ struct DpCtx {
     int maxn;
     int cur;             // which half of dist holds the last completed layer
     int layer;           // lattice layer of the last completed step
-    int tie;             // an equal-cost alternative was seen (igraph's pick then depends on heap order)
+    int tie;             // some node's final (cost, own distance) minimum has two in-edges (igraph's pick then depends
+                         // on heap order)
     int snap_li;         // step whose result dsave holds (0: no snapshot)
     int tie_save;        // tie flag at the snapshot
     int fe0, fe1, fe2;   // stateful tick: edges of the last solution whose cost is scaled (GLNT:155-162), -1: none
@@ -246,6 +247,7 @@ __device__ __forceinline__ int dp_run(const LatDev& lt, int lane, DpCtx& c, int 
         for (int j = lane; j < maxn; j += 32) {
             double best = LTPL_INF, best_ds = LTPL_INF;
             int best_k = 255;   // start-layer node index of the chosen in-edge (255: unreachable)
+            int tie_here = 0;   // the current (best, best_ds) is attained by a second in-edge
             bool present = j < nl && !(nxt == rem_layer && j >= rem_lo && j < rem_hi);
             if (ZONE && present && zs) present = !((zs[(nbase + j) >> 5] >> ((nbase + j) & 31)) & 1u);
             if (present) {
@@ -268,8 +270,9 @@ __device__ __forceinline__ int dp_run(const LatDev& lt, int lane, DpCtx& c, int 
                         best = alt;
                         best_ds = ds;
                         best_k = r.src;
+                        tie_here = 0;
                     } else if (alt == best && ds == best_ds) {
-                        tie = 1;
+                        tie_here = 1;
                     }
                 };
                 // in-edges in CSC order (igraph's relaxation order); nodes with many in-edges keep two records in flight
@@ -283,6 +286,7 @@ __device__ __forceinline__ int dp_run(const LatDev& lt, int lane, DpCtx& c, int 
                 #pragma unroll 1
                 for (; k < io.y; ++k) relax(lt.edge_rec[io.x + k], io.x + k);
             }
+            tie |= tie_here;
             dnxt[j] = best;
             c.pred[li * maxn + j] = (unsigned char)best_k;
             any |= (best_k != 255);
@@ -333,7 +337,7 @@ __device__ __forceinline__ int dp_run_pair(const LatDev& lt, int lane, DpCtx& c,
         const double* dcur = c.dist + cur * maxn + hoff;
         double* dnxt = c.dist + (cur ^ 1) * maxn + hoff;
         double best = LTPL_INF, best_ds = LTPL_INF;
-        int best_k = 255;
+        int best_k = 255, tie_here = 0;
         bool present = j < nl && !(nxt == rem_layer && (half ? (j < split) : (j >= split)));
         if (ZONE && present && zs) present = !((zs[(nbase + j) >> 5] >> ((nbase + j) & 31)) & 1u);
         if (present) {
@@ -359,11 +363,13 @@ __device__ __forceinline__ int dp_run_pair(const LatDev& lt, int lane, DpCtx& c,
                     best = alt;
                     best_ds = ds;
                     best_k = r.src;
+                    tie_here = 0;
                 } else if (alt == best && ds == best_ds) {
-                    tie = 1;
+                    tie_here = 1;
                 }
             }
         }
+        tie |= tie_here;
         dnxt[j] = best;
         c.pred[li * maxn + lane] = (unsigned char)best_k;
         const unsigned alive = __ballot_sync(LTPL_FULL, best_k != 255);
@@ -414,6 +420,7 @@ __device__ __forceinline__ int dp_goal(const LatDev& lt, int lane, const DpCtx& 
             best = alt;
             best_ds = ds;
             best_j = j;
+            tie = 0;   // a tie with a candidate this lane has since beaten does not count
         } else if (alt == best && ds == best_ds) {
             tie = 1;
         }
@@ -432,6 +439,7 @@ __device__ __forceinline__ int dp_goal(const LatDev& lt, int lane, const DpCtx& 
     in = in && ((unsigned)ud == dl) && (best < LTPL_INF);
     const unsigned win = __ballot_sync(LTPL_FULL, in);
     const unsigned gj = __reduce_min_sync(LTPL_FULL, in ? (unsigned)best_j : 0x7fffffffu);
+    // tie: the minimum is attained by several goal-layer nodes, across lanes or within a winning lane
     if (__popc(win) > 1 || __any_sync(LTPL_FULL, tie && in)) *tie_out = 1;
     return (int)gj;
 }

@@ -44,7 +44,10 @@ extern "C" {
 /* status bits per (scenario, slot) */
 #define LTPL_ST_FOUND            (1 << 0)  /* a path exists for this slot (MOPG:246-257)                               */
 #define LTPL_ST_REDUCED_HORIZON  (1 << 1)  /* goal layer was moved towards the vehicle (MOPG:203-243)                  */
-#define LTPL_ST_TIE_AMBIGUOUS    (1 << 2)  /* exact cost tie met in the search: igraph's pick is heap-order dependent  */
+#define LTPL_ST_TIE_AMBIGUOUS    (1 << 2)  /* some node of the search, or its virtual goal, has its final (cost, own
+                                              distance) minimum attained by >= 2 candidates (in-edges / goal-layer
+                                              nodes); igraph's pick there is heap-order dependent. Ties that a later
+                                              candidate beats do not count                                          */
 #define LTPL_ST_START_BLOCKED    (1 << 3)  /* start node removed by the action's node filter (GB:882-885)              */
 #define LTPL_ST_TRAJ_VALID       (1 << 4)  /* trajectory kept in the action set after calc_vel_profile (OTH:945-948)   */
 #define LTPL_ST_VEL_BOUND_VIOL   (1 << 5)  /* |vx[0] - vel_plan| >= v_max_offset or follow-mode bound broken (OTH:907)  */

@@ -346,6 +346,9 @@ class OracleLTPL(object):
 
         nodes [removed_lo, removed_hi) of `removed_layer` are absent (MOPG:148-159); `blocked` = edge ids removed from
         the active filter (None for the un-blocked 'planning_range' graph); cost_factor = {edge id: factor} (GB:478-512).
+        tie_flag: some node of the search, or its virtual goal, has its final (cost, own distance) minimum attained by
+        two or more candidates (in-edges of a node, goal-layer nodes of the goal); ties a later candidate beats do not
+        count.
         """
         lt = self.lat
         sl, sn = start_node
@@ -378,6 +381,7 @@ class OracleLTPL(object):
                 best = inf
                 best_ds = inf
                 best_i = -1
+                tie_here = False
                 for e in range(e0, e0 + cnt):
                     i = int(lt.edge_src[e])
                     ds = dist.get(i)
@@ -389,8 +393,10 @@ class OracleLTPL(object):
                     alt = ds + c
                     if alt < best or (alt == best and ds < best_ds):
                         best, best_ds, best_i = alt, ds, i
+                        tie_here = False
                     elif alt == best and ds == best_ds:
-                        tie = True
+                        tie_here = True
+                tie = tie or tie_here
                 if best_i >= 0:
                     nd[j] = best
                     par[j] = best_i
@@ -403,12 +409,15 @@ class OracleLTPL(object):
         best = inf
         best_ds = inf
         best_j = -1
+        tie_here = False
         for j in sorted(dist):
             alt = dist[j] + abs(rl - j) * lt.lat_resolution * lt.virt_goal_node_cost
             if alt < best or (alt == best and dist[j] < best_ds):
                 best, best_ds, best_j = alt, dist[j], j
+                tie_here = False
             elif alt == best and dist[j] == best_ds:
-                tie = True
+                tie_here = True
+        tie = tie or tie_here
         seq = [best_j]
         for par in reversed(parents):
             seq.append(par[seq[-1]])
